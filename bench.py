@@ -24,6 +24,9 @@ with N (the N-fold periodic supercell of the N = 1 frame along x: N x 10 648 ato
 10 648-atom frame.  `checks`: sum of all forces = 0, and in halo mode `partition_parity` = forces / energy of the
 sharded frame against the UNSHARDED base frame evaluated on each rank (every atom is a periodic copy of a base atom).
 `--decomp frames` keeps the round-1 mode (one independent frame per GPU, the reference's DDP axis).
+`--dump-outputs DIR`: after the timed steps, the floating-point outputs of the last timed step (total_energy, forces;
+the reference arm also atomic_energy) are written as DIR/<name>.npy (float32 / float64; `.rank<r>` before `.npy` when
+N > 1).  Inputs and weights are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -202,8 +205,10 @@ def run_reference(args, rank, world):
         omodel.energy_and_forces(sd, cfg, sysd, torch.float32, tp_chunk=chunk)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        omodel.energy_and_forces(sd, cfg, sysd, torch.float32, tp_chunk=chunk)
+        e, ea, f = omodel.energy_and_forces(sd, cfg, sysd, torch.float32, tp_chunk=chunk)
     dt = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:
+        dump_outputs(output_arrays({"total_energy": e, "atomic_energy": ea, "forces": f}), args.dump_outputs)
     val = n_atoms / dt
     sample = (f"{n_atoms}-atom {WORKLOADS[args.workload][0]} box, same model/density, E={sysd['edge_index'].shape[1]}, "
               f"edge chunk {chunk}, {cores} of {os.cpu_count()} host threads (fastest of a short sweep)")
@@ -388,6 +393,41 @@ def halo_exchange_profile(dims, plan, halo, dev, world, reps=10):
     return out
 
 
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
+
+
+def output_arrays(out, exclude=()):
+    """Host copies of the floating-point tensors of one step's result dict (keys in ``exclude``, the step's inputs,
+    are skipped), as float32 / float64 numpy arrays."""
+    arrs = {}
+    for k, v in out.items():
+        if k in exclude or not torch.is_tensor(v) or not v.is_floating_point():
+            continue
+        v = v.detach()
+        if v.dtype not in (torch.float32, torch.float64):
+            v = v.float()
+        arrs[k] = v.cpu().numpy().copy()
+    return arrs
+
+
+def dump_outputs(arrs, out_dir, suffix=""):
+    """``out_dir/<name><suffix>.npy`` for every array, DUMP_LIMIT_BYTES in all: an array over its share of the limit
+    is replaced by a fixed seeded sample of its flattened elements, with their flat positions (float64) in
+    ``<name><suffix>.index.npy``."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_LIMIT_BYTES // max(1, len(arrs))
+    for name, a in sorted(arrs.items()):
+        if a.nbytes > share:
+            flat = a.reshape(-1)
+            keep = share // (a.itemsize + 8)
+            idx = np.sort(np.random.default_rng(0).choice(flat.size, keep, replace=False))
+            np.save(os.path.join(out_dir, f"{name}{suffix}.index.npy"), idx.astype(np.float64))
+            a = flat[idx]
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), a)
+
+
 def _time_cuda(fn, reps):
     for _ in range(3):
         fn()
@@ -552,7 +592,12 @@ def main():
     ap.add_argument("--profile-step", action="store_true",
                     help="run one warm-up step, then ONE step between cudaProfilerStart/Stop (for ncu "
                          "--profile-from-start off); prints no bench line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the floating-point outputs of the last timed step as DIR/<name>.npy (float32/float64, "
+                         "at most 64 MB in all; a larger output is replaced by a fixed seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -699,7 +744,7 @@ def main():
         n0 = _capi.launch_count()
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record()
         torch.cuda.synchronize()
         if world > 1:
@@ -712,7 +757,7 @@ def main():
             t = torch.tensor([ms], dtype=torch.float64, device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms, launches
+        return ms, launches, out
 
     if args.profile_step:
         step_resident()
@@ -726,11 +771,14 @@ def main():
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms_res, launches = timed(step_resident, args.steps, args.warmup)
-    ms_e2e, _ = timed(step_e2e, args.steps, 1)
+    ms_res, launches, last = timed(step_resident, args.steps, args.warmup)
+    if args.dump_outputs:  # host copies now: the replays of the e2e legs below overwrite the graph's output buffers
+        dump_outputs(output_arrays(last, exclude=resident), args.dump_outputs, f".rank{rank}" if world > 1 else "")
+    del last
+    ms_e2e, _, _ = timed(step_e2e, args.steps, 1)
     ms_e2e_nl = None
     if world == 1 and "cell" in sysd:
-        ms_e2e_nl, _ = timed(step_e2e_device_nl, args.steps, 1)
+        ms_e2e_nl, _, _ = timed(step_e2e_device_nl, args.steps, 1)
     clocks = sampler.stop() if rank == 0 else None
     if graphed is not None:
         graphed.check_sorted()  # the in-graph "edges grouped by destination" flag of the last replay

@@ -173,8 +173,10 @@ __device__ __forceinline__ void preact4(const float (&x)[NB], const float2 (&w01
   }
 }
 
+// kLo: also write the tf32 low parts of h to h_lo (as k_hidden_fwd does); h itself is the same either way
+template <bool kLo>
 __global__ void __launch_bounds__(256) k_hidden_fwd2(const float* __restrict__ emb, const float* __restrict__ W1s,
-                                                     int64_t E, float* __restrict__ h) {
+                                                     int64_t E, float* __restrict__ h, float* __restrict__ h_lo) {
   const int lane = threadIdx.x & 31, m0 = lane * 4;
   float2 w01[NB], w23[NB];
 #pragma unroll
@@ -199,12 +201,15 @@ __global__ void __launch_bounds__(256) k_hidden_fwd2(const float* __restrict__ e
       bcast_basis(cur, j, x);
       float2 p01, p23;
       preact4(x, w01, w23, p01, p23);
-      float4 o;
-      o.x = p01.x * sigmoid_v2(p01.x);
-      o.y = p01.y * sigmoid_v2(p01.y);
-      o.z = p23.x * sigmoid_v2(p23.x);
-      o.w = p23.y * sigmoid_v2(p23.y);
+      float4 o;  // __fmul_rn: no FMA contraction into tf32_lo's subtraction, h_lo is the low part of the stored h
+      o.x = __fmul_rn(p01.x, sigmoid_v2(p01.x));
+      o.y = __fmul_rn(p01.y, sigmoid_v2(p01.y));
+      o.z = __fmul_rn(p23.x, sigmoid_v2(p23.x));
+      o.w = __fmul_rn(p23.y, sigmoid_v2(p23.y));
       __stcs(reinterpret_cast<float4*>(hrow + (int64_t)j * H), o);
+      if (kLo)
+        __stcs(reinterpret_cast<float4*>(h_lo + e0 * H + m0 + (int64_t)j * H),
+               make_float4(tf32_lo(o.x), tf32_lo(o.y), tf32_lo(o.z), tf32_lo(o.w)));
     }
     cur = nxt;
   }
@@ -322,7 +327,7 @@ extern "C" int nqb_mlp_hidden_set_variant(int variant) {  // returns the previou
 // its next batch is always prefetched; fewer CTAs when there are fewer batches than warps
 template <typename K>
 static unsigned hidden_grid2(K kernel, int which, int64_t E) {
-  static int ctas_dev[2][64] = {{0}, {0}};
+  static int ctas_dev[3][64] = {{0}, {0}, {0}};
   int dev = 0;
   cudaGetDevice(&dev);
   dev &= 63;
@@ -343,8 +348,11 @@ extern "C" int nqb_mlp_hidden_fwd(const float* emb, const float* W1s, int64_t E,
   if (E == 0) return 0;
   if (!emb || !W1s || !h) return nqb_set_error("nqb_mlp_hidden_fwd: null pointer");
   const int64_t threads = E * 32;
+  // the variant alone picks the kernel: asking for h_lo must not change h
   if (hidden_variant() == 2 && h_lo == nullptr)
-    k_hidden_fwd2<<<hidden_grid2(k_hidden_fwd2, 0, E), 256, 0, (cudaStream_t)st>>>(emb, W1s, E, h);
+    k_hidden_fwd2<false><<<hidden_grid2(k_hidden_fwd2<false>, 0, E), 256, 0, (cudaStream_t)st>>>(emb, W1s, E, h, nullptr);
+  else if (hidden_variant() == 2)
+    k_hidden_fwd2<true><<<hidden_grid2(k_hidden_fwd2<true>, 2, E), 256, 0, (cudaStream_t)st>>>(emb, W1s, E, h, h_lo);
   else
     k_hidden_fwd<<<hidden_grid(threads), 256, 0, (cudaStream_t)st>>>(emb, W1s, E, h, h_lo);
   nqb_count_launch();

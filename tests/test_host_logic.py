@@ -297,16 +297,17 @@ def test_reference_checkpoint_key_mapping_round_trip():
         load_reference_state_dict(b, {"func.type_embed.embed_module.weight": torch.zeros(3, 3)}, strict=False)
 
 
-def test_bench_reference_arm_json_contract():
-    """``bench.py --impl reference`` (the CPU arm the driver times beside the GPU arm): one JSON line with the metric /
+def test_bench_reference_arm_json_contract(tmp_path):
+    """``bench.py --impl reference`` (the CPU arm timed beside the GPU arm): one JSON line with the metric /
     unit / higher_is_better of the own arm, ``impl``, a ``cpu_baseline`` describing the run, zero-copy ``e2e`` and the
-    workload + model keys in ``config``."""
+    workload + model keys in ``config``; ``--dump-outputs`` writes the outputs of its last step."""
     import json
     import subprocess
     import sys
 
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--workload", "tiny",
-                        "--steps", "1", "--warmup", "0"], capture_output=True, text=True, timeout=600)
+                        "--steps", "1", "--warmup", "0", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
     line = json.loads(r.stdout.strip().splitlines()[-1])
     assert line["impl"] == "reference" and line["metric"] == "atom-steps/sec (energy+forces)"
@@ -317,6 +318,9 @@ def test_bench_reference_arm_json_contract():
     cfg = line["config"]
     assert cfg["workload"] == "tiny" and cfg["l_max"] == 2 and cfg["num_layers"] == 3 and cfg["num_features"] == 8
     assert cfg["atoms_per_step_sample"] > 0 and cfg["edges_per_step_sample"] > 0
+    f = np.load(tmp_path / "forces.npy")
+    assert f.shape == (cfg["atoms_per_step_sample"], 3) and f.dtype in (np.float32, np.float64)
+    assert np.load(tmp_path / "total_energy.npy").size == 1 and (tmp_path / "atomic_energy.npy").exists()
 
 
 def test_bench_cpu_sample_size_respects_the_budget():
@@ -351,3 +355,31 @@ def test_bench_force_sum_property_vector():
     # two "ranks" whose forces cancel
     tot = bench.force_sum_vector(f) + bench.force_sum_vector(-f)
     assert float(tot[:3].abs().max()) == 0.0 and float(tot[4]) == 2.0
+
+
+def test_bench_dump_outputs(tmp_path):
+    """``bench.py --dump-outputs``: the floating-point outputs of a step (not its inputs, not integer flags) as float32 /
+    float64 .npy files, 64 MB in all, a larger array replaced by the same seeded sample on every run."""
+    import importlib.util
+
+    spec = importlib.util.spec_from_file_location("nqb_bench3", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    out = {"total_energy": torch.tensor([1.5], dtype=torch.float64), "forces": torch.randn(7, 3),
+           "atomic_energy": torch.randn(7, 1, dtype=torch.float16), "edges_sorted": torch.ones(1, dtype=torch.int32),
+           "pos": torch.randn(7, 3, dtype=torch.float64)}
+    arrs = bench.output_arrays(out, exclude={"pos": None})
+    assert sorted(arrs) == ["atomic_energy", "forces", "total_energy"]
+    assert arrs["forces"].dtype == np.float32 and arrs["total_energy"].dtype == np.float64
+    assert arrs["atomic_energy"].dtype == np.float32
+    bench.dump_outputs(arrs, str(tmp_path / "a"))
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "forces.npy"), out["forces"].numpy())
+    assert np.load(tmp_path / "a" / "total_energy.npy").tolist() == [1.5]
+    # over the limit: a seeded sample of the flattened elements and their positions
+    big = {"x": np.arange(bench.DUMP_LIMIT_BYTES // 8 + 1000, dtype=np.float64), "e": np.zeros(1)}
+    for d in ("b", "c"):
+        bench.dump_outputs(big, str(tmp_path / d), suffix=".rank1")
+    x, idx = np.load(tmp_path / "b" / "x.rank1.npy"), np.load(tmp_path / "b" / "x.rank1.index.npy")
+    assert idx.dtype == np.float64 and x.dtype == np.float64 and np.array_equal(x, idx) and 0 < x.size < big["x"].size
+    assert np.array_equal(idx, np.load(tmp_path / "c" / "x.rank1.index.npy"))
+    assert sum(f.stat().st_size for f in (tmp_path / "b").iterdir()) <= bench.DUMP_LIMIT_BYTES
